@@ -17,7 +17,13 @@ One "step" = one pass of the hot path over the whole batch.  `value` is measured
 on the launch stream, profiling off); `roofline` comes from a separate profiled pass; `e2e` goes through the public API with
 host arrays, host->device and device->host copies (and the gather) inside the timed region.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload sweep|mc65536]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload sweep|mc65536] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step computed (z, obj, kkt, iters, status and, for the sweep, the minimum trip
+time of every instance) as DIR/<name>.npy in float64, rows in the batch's instance order, `instance` naming each row's index in
+the batch (under torchrun every rank writes its share, prefixed rank<r>_).  Rows of instances flagged infeasible (status 4) are
+zero but for their status.  The inputs are fixed by the arguments, so two builds can be compared output for output.  The files
+stay under 64 MB; a larger batch (mc65536) is represented by a fixed, seeded sample of its instances.
 """
 import argparse
 import json
@@ -41,6 +47,7 @@ OPTS = {'numIntervals': N_INT, 'maxIterations': 500, 'integrationMethod': 'RK',
         'integrationOptions': {'order': 4, 'numSteps': 1, 'numApproxSteps': 1}}
 TMIN_REF = 1035.5536      # restatement-derived (SURVEY appendix E); re-derived on the device in every step
 METRIC = 'OCP solves/sec (batched, 1/2/4/8 B200) vs CasADi+IPOPT on host cores'
+DUMP_BYTES = (64 << 20) - (1 << 20)      # --dump-outputs stays under 64 MB with room for the .npy headers
 
 
 def sweep_times(n, tmin=TMIN_REF):
@@ -206,10 +213,10 @@ class Resident:
     """One rank's share of a batch with its inputs resident in HBM: parameter planes in dealt (stream-pool) order, track
     tables, result buffers; `step()` runs the hot path once (optionally with the concurrent minimum-time presolve)."""
 
-    def __init__(self, solver, dev, streams, lanes, T, overrides=None, lossT=0.0, lossR=0.0, presolve=False):
+    def __init__(self, solver, dev, streams, lanes, T, overrides=None, lossT=0.0, lossR=0.0, presolve=False, name=''):
         import torch
         from mseetc import _cabi
-        self.torch, self.cabi, self.solver, self.dev = torch, _cabi, solver, dev
+        self.torch, self.cabi, self.solver, self.dev, self.name = torch, _cabi, solver, dev, name
         n = self.n = len(T)
         zero = np.zeros(n)
         overrides = dict(overrides or {})
@@ -289,6 +296,22 @@ class Resident:
                 t['ms'] += v['ms']; t['launches'] += v['launches']; t['cells'] += v['cells']; t['bytes_per_cell'] = v['bytes_per_cell']
 
 
+def dump_outputs(dirname, parts, budget, seed=20260101):
+    """Writes DIR/<prefix><key>.npy (float64) for parts [(prefix, instance indices, {key: array with one row per instance})].
+    If they exceed `budget` bytes, every part keeps the same fixed, seeded fraction of its rows; <prefix>instance.npy holds the
+    batch index of every row written."""
+    parts = [(p, np.asarray(idx, dtype=np.float64), {k: np.asarray(a, dtype=np.float64) for k, a in arrs.items()}) for p, idx, arrs in parts]
+    total = sum(idx.nbytes + sum(a.nbytes for a in arrs.values()) for _, idx, arrs in parts)
+    frac = min(1.0, budget / total)
+    rng = np.random.default_rng(seed)
+    os.makedirs(dirname, exist_ok=True)
+    for prefix, idx, arrs in parts:
+        n = len(idx)
+        rows = np.arange(n) if frac == 1.0 else np.sort(rng.choice(n, max(1, int(n * frac)), replace=False))
+        for k, a in dict(arrs, instance=idx).items():
+            np.save(os.path.join(dirname, prefix + k + '.npy'), a[rows])
+
+
 def mc_recipe(train):
     "SURVEY.md 8(d) config 3: per-instance train parameters, first half constant efficiencies, second half spline loss map."
     rng = np.random.default_rng(20260101)
@@ -354,10 +377,12 @@ def run_gpu(args):
         if len(sel):
             o = {k: v[sel] for k, v in ov.items()}
             etaT, etaR = o.pop('etaTraction'), o.pop('etaRgBrake')
-            residents.append((Resident(ssolver, dev, args.streams, lanes, T[sel], overrides=o, lossT=(1 - etaT) / etaT, lossR=1 - etaR), sel))
+            residents.append((Resident(ssolver, dev, args.streams, lanes, T[sel], overrides=o, lossT=(1 - etaT) / etaT, lossR=1 - etaR,
+                                       name='constant_'), sel))
         sel = idx[idx >= 32768]
         if len(sel):
-            residents.append((Resident(dsolver, dev, args.streams, lanes, T[sel], overrides={k: v[sel - 32768] for k, v in ov2.items()}), sel))
+            residents.append((Resident(dsolver, dev, args.streams, lanes, T[sel], overrides={k: v[sel - 32768] for k, v in ov2.items()},
+                                       name='lossmap_'), sel))
         partition = 'ranges'
 
     def step():
@@ -396,6 +421,20 @@ def run_gpu(args):
     ms, outs = timed(step, args.steps)
     launches = sum(r.launches for r, _ in residents)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # the result buffers are reused by every later pass: copy out what the last timed step left in them
+        parts = []
+        for (r, sel), out in zip(residents, outs):
+            arrs = {k: out[k].cpu().numpy()[r.back] for k in ('z', 'obj', 'kkt', 'iters', 'status')}
+            # an instance flagged infeasible stops at whichever iteration the concurrent minimum-time presolve reaches it, which
+            # varies from run to run: its rows are blanked (the public API blanks the trajectory of a failed solve as well)
+            flagged = arrs['status'] == 4
+            for k in ('z', 'obj', 'kkt', 'iters'):
+                arrs[k][flagged] = 0
+            if r.ht is not None:
+                arrs['tmin'] = r.tmin_dev.cpu().numpy()[r.back]
+            parts.append(('%s%s' % ('rank%d_' % rank if world > 1 else '', r.name), sel, arrs))
+        dump_outputs(args.dump_outputs, parts, DUMP_BYTES // world)
 
     # what was solved (this rank), then summed over the ranks
     stats = dict(instances=0, feasible=0, converged=0, flagged=0, failed=0, iters_sum=0.0, iters_max=0, ticks=0)
@@ -606,7 +645,13 @@ def main():
     ap.add_argument('--no-latency', action='store_true', help='skip the config-1 single-solve latency leg')
     ap.add_argument('--streams', type=int, default=1, help='concurrent sub-batches (CUDA streams / host threads) per GPU')
     ap.add_argument('--sweep-lanes', default='auto', help="Riccati sweeps: 1 sequential, 8/16/32 parallel in time, 'auto'")
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the results of the last timed step as DIR/<name>.npy (float64, '
+                                                          'at most 64 MB: a seeded sample of the instances of a larger batch)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the results of the GPU arm; the reference arm keeps none')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -4,7 +4,7 @@ A restatement (numpy / scipy / sympy, FP64) of the NLP that the reference
 builds in ``mseetc/ocp.py:80-307`` and hands to CasADi+IPOPT at ``ocp.py:290,359``.
 The algorithm that actually solves the NLP in the reference lives in the
 un-vendored third-party wheel ``casadi==3.6.3`` (``setup.py:11``; bundles IPOPT 3.14 +
-MUMPS), which is absent from ``/root/reference`` and from this image.  The oracle
+MUMPS), which the reference repository does not contain.  The oracle
 therefore restates IPOPT's *published* algorithm (Waechter & Biegler 2006,
 "On the implementation of an interior-point filter line-search algorithm for
 large-scale nonlinear programming") on the reference's exact variable/row layout.

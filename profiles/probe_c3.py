@@ -1,5 +1,6 @@
 import os, sys
-sys.path[:0] = ['/root/repo', '/root/repo/ms-eetc_b200', '/root/repo/profiles']
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path[:0] = [ROOT, os.path.join(ROOT, 'ms-eetc_b200'), os.path.join(ROOT, 'profiles')]
 import numpy as np
 import __graft_entry__ as ge
 ge.build()

@@ -1,5 +1,5 @@
 import sys, os
-ROOT='/root/repo'
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0]=[ROOT, ROOT+'/ms-eetc_b200']
 import numpy as np, torch
 import __graft_entry__ as ge
