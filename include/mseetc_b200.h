@@ -176,7 +176,7 @@ int mseetc_postprocess_batch(mseetc_handle h, int32_t n_instances, const double*
 int mseetc_set_sweep_lanes(mseetc_handle h, int lanes);
 int mseetc_last_sweep_lanes(mseetc_handle h);          /* lanes the last mseetc_solve_batch on h ran with */
 /* compaction passes launched in the last solve (running instances moved into the slots of finished ones so that they fill whole
- * warps; csrc/compact.cuh; results do not depend on it; MSEETC_COMPACT=0 switches it off) */
+ * warps; csrc/compact.cuh; results do not depend on it; mseetc_set_compaction(h, 0) switches it off) */
 int mseetc_last_compactions(mseetc_handle h);
 int mseetc_last_compaction_moves(mseetc_handle h);     /* instances moved by those passes */
 int mseetc_set_compaction(mseetc_handle h, int on);

@@ -10,7 +10,6 @@
 #include <algorithm>
 #include <cstdio>
 #include <limits>
-#include <cstdlib>
 #include <cstring>
 #include <new>
 #include <string>
@@ -32,28 +31,19 @@ thread_local std::string g_err;
 
 
 // ---- interval-parallel kernels: one thread per (interval k, instance), warp = 32 instances at one k.  The kernels stride over
-// the cells, so any grid works; the default is one block per 128 cells (measured faster than a persistent grid of a few blocks
-// per SM, MSEETC_CELL_WAVES=w selects the latter for experiments: 110.9k / 115.5k / 118.6k / 122.0k solves/s at w = 1/2/4/8
-// against 122.6k with the full grid on the bench workload).
+// the cells, so any grid works; they are launched with one block per 128 cells (measured faster than a persistent grid of a few
+// blocks per SM: 110.9k / 115.5k / 118.6k / 122.0k solves/s with 1/2/4/8 waves against 122.6k with the full grid on the bench
+// workload).
 // (MS_CELL_KERNEL: variants.h)
-#ifndef MS_MINB_TRIAL
-#define MS_MINB_TRIAL 2
-#endif
-#ifndef MS_MINB_EVAL
-#define MS_MINB_EVAL 2
-#endif
-#ifndef MS_MINB_STEP
-#define MS_MINB_STEP 3
-#endif
 MS_CELL_KERNEL(k_cell_setup, 4, cell_setup(c, io, k, s))
 MS_CELL_KERNEL(k_cell_init, 4, cell_init<false>(c, k, s))
 // k_cell_trial_eval: the interval evaluation AT THE TRIAL POINT, which it forms on the way (one kernel per iteration instead of
 // trial + evaluation); k_cell_eval: the same at the current iterate, once per solve for the starting point
-MS_CELL_KERNEL(k_cell_trial_eval, MS_MINB_TRIAL, (cell_eval<false, true>(c, k, s)))
-MS_CELL_KERNEL(k_cell_eval, MS_MINB_EVAL, (cell_eval<false, false>(c, k, s)))
+MS_CELL_KERNEL(k_cell_trial_eval, 2, (cell_eval<false, true>(c, k, s)))
+MS_CELL_KERNEL(k_cell_eval, 2, (cell_eval<false, false>(c, k, s)))
 // (the variants with the spline loss map, the collocation integrator and integrated losses live in variants_*.cu: further translation units that
 // compile next to this one, launched through mseetc::launch_variant)
-MS_CELL_KERNEL(k_cell_step, MS_MINB_STEP, cell_step<false>(c, k, s))
+MS_CELL_KERNEL(k_cell_step, CELL_STEP_MINB, cell_step<false>(c, k, s))
 MS_CELL_KERNEL(k_cell_extract, 4, cell_extract(c, io, k, s))
 
 __global__ void __launch_bounds__(64) k_inst_setup(Ctx c, BatchIO io) {
@@ -81,10 +71,7 @@ __global__ void __launch_bounds__(128) k_inst_profile(Ctx c, int useSmem) {
 // running instances has only 64 tiles: one block per tile left 84 of the 148 SMs idle in these latency-bound kernels.
 // `mirror` (mapped pinned host memory): the completion counter as it stands when this kernel runs, for the host's polling --
 // a store from the kernel instead of a 4-byte cudaMemcpyAsync between two kernels of every tick (which cost ~10 us of stream time)
-#ifndef MS_RED_CL
-#define MS_RED_CL 4
-#endif
-enum { RED_CL = MS_RED_CL, RED_WB = RED_W / RED_CL };      // blocks per cluster, warps per block
+enum { RED_CL = 4, RED_WB = RED_W / RED_CL };      // blocks per cluster, warps per block
 static_assert(RED_W % RED_CL == 0, "cluster size must divide the interleave factor");
 __device__ __forceinline__ const double* cluster_peer(const double* p, unsigned rank) {
     return cooperative_groups::this_cluster().map_shared_rank(p, rank);
@@ -167,11 +154,7 @@ __global__ void __cluster_dims__(RED_CL, 1, 1) __launch_bounds__(32 * RED_WB) k_
 
 // Riccati sweeps: one thread per instance, stage data prefetched `depth` intervals ahead through a cp.async ring
 // in dynamic shared memory ((depth+1) * RING_NF_MAX * blockDim doubles).
-// BULK = true (experiment, MSEETC_STEP_BULK=1): tiles whose running instances share one interval count fetch their stage data
-// with bulk copies of the TMA unit (cp.async.bulk + mbarrier, BulkRing) instead of per-lane cp.async.  Measured on B200:
-// 244 us per launch against 178 us -- in this one-warp, latency-bound recursion the mbarrier wait and the warp barrier per
-// interval cost more than the 23 + 14 LDGSTS they replace -- so the per-lane ring is the default.
-template <int BS, int DEPTH, bool BULK>
+template <int BS, int DEPTH>
 __global__ void __launch_bounds__(BS) k_step(Ctx c) {
     extern __shared__ __align__(128) double ring[];
     const int s = blockIdx.x * BS + threadIdx.x;
@@ -179,21 +162,6 @@ __global__ void __launch_bounds__(BS) k_step(Ctx c) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const bool active = s < c.cfg.nInst && c.I(SI_PHASE, s) == PH_FACTOR;
     double* wring = ring + (size_t)warp * ((DEPTH + 1) * RING_NF_MAX * 32);
-    if (BULK) {
-        const unsigned mask = __ballot_sync(0xffffffffu, active);
-        if (!active) return;
-        const int N = c.I(SI_N_INT, s);
-        if (__all_sync(mask, N == __shfl_sync(mask, N, __ffs((int)mask) - 1))) {
-            unsigned long long* bars = reinterpret_cast<unsigned long long*>(ring + (size_t)(BS / 32) * ((DEPTH + 1) * RING_NF_MAX * 32))
-                                       + (size_t)warp * 2 * (DEPTH + 1);
-            BulkRing<BwdFields, DEPTH> fb;
-            BulkRing<FwdFields, DEPTH> ff;
-            fb.setup(wring, bars, mask, lane);
-            ff.setup(wring, bars + (DEPTH + 1), mask, lane);
-            inst_step_warp(c, s, mask, fb, ff);
-            return;
-        }
-    }
     if (!active) return;
     // every lane prefetches its own intervals (cp.async, one column per lane): works for mixed interval counts inside a tile
     RingFetch<BwdFields, 32, DEPTH> fb;
@@ -209,10 +177,8 @@ __global__ void __launch_bounds__(BS) k_step(Ctx c) {
 // shared memory; the two short sequential chains over the chunks are run by the lane of chunk 0.  Stage data are prefetched
 // through the same per-thread cp.async ring as in k_step.  An instance whose element algebra fails, or whose chain and recursion
 // disagree, is redone by the sequential sweeps (lane of chunk 0, same kernel), so accuracy never rests on the chain.
-// L2 prefetch distance of the sweep rings, in intervals beyond the ring's own look-ahead (0 = off; 104 -> 95 us with 3)
-#ifndef MS_PIT_PF
-#define MS_PIT_PF 3
-#endif
+// L2 prefetch distance of the sweep rings, in intervals beyond the ring's own look-ahead (none: 104 us, 3: 95 us)
+enum { PIT_PF = 3 };
 template <int SL, int G, int DEPTH>
 __global__ void __launch_bounds__(SL * G) k_step_pit(Ctx c, int* fallbackCount) {
     extern __shared__ __align__(128) double pit_sm[];
@@ -234,12 +200,12 @@ __global__ void __launch_bounds__(SL * G) k_step_pit(Ctx c, int* fallbackCount) 
     pit_chunk(t.N, G, l, t.kLo, t.kHi);
     if (active) pit_read_reference(c, t);
     if (l == 0) flags[col] = 0;
-    RingFetch<BwdFields, BS, DEPTH, MS_PIT_PF> fb;
+    RingFetch<BwdFields, BS, DEPTH, PIT_PF> fb;
     fb.sm = ring + threadIdx.x;
     // the forward sweep spends next to no arithmetic per interval: it needs the deeper look-ahead, and its 14 planes per interval
     // leave room for it in the same ring
     constexpr int FDEPTH = ((DEPTH + 1) * BwdFields::NF) / FwdFields::NF - 1;
-    RingFetch<FwdFields, BS, FDEPTH, 2 * MS_PIT_PF> ff;
+    RingFetch<FwdFields, BS, FDEPTH, 2 * PIT_PF> ff;
     ff.sm = ring + threadIdx.x;
     double delta = 0.0;
     bool pending = active, failed = false, fallback = false;
@@ -605,7 +571,7 @@ int mseetc_solve_batch(mseetc_handle h, int32_t n, const double* params, const i
     BatchIO io{params, nint, trk_of, trk_off, ds, c0, bmax, tmin, z_out, lam_out, obj, kkt, iters, status};
 
     const size_t cellThreads = (size_t)g.NK * g.S;
-    const unsigned cgridFull = (unsigned)((cellThreads + 127) / 128);
+    const unsigned cgrid = (unsigned)((cellThreads + 127) / 128);      // grid of the interval kernels (see MS_CELL_KERNEL)
     const int ib = (g.S >= 148 * 64 * 2) ? 64 : 32;
     const unsigned igrid = (unsigned)((g.S + ib - 1) / ib);
     // prefetch depth of the Riccati ring: as deep as shared memory allows for the blocks resident on one SM
@@ -615,41 +581,30 @@ int mseetc_solve_batch(mseetc_handle h, int32_t n, const double* params, const i
         cudaGetDevice(&devId);
         cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, devId);
     }
-    // grids of the interval kernels (see MS_CELL_KERNEL)
-    static const int cellWaves = []() { const char* e = getenv("MSEETC_CELL_WAVES"); return e ? atoi(e) : 0; }();
-    auto pgrid = [&](int minb) {
-        if (cellWaves < 1) return cgridFull;
-        const unsigned want = (unsigned)(nsm * minb * cellWaves) | 1u;
-        return want < cgridFull ? want : cgridFull;
-    };
-    const unsigned cgrid = pgrid(4), gridTrial = pgrid(dyn ? 2 : MS_MINB_TRIAL), gridEval = pgrid(dyn ? 2 : MS_MINB_EVAL), gridStep = pgrid(MS_MINB_STEP), gridIrk = pgrid(1);
     const int blocksPerSm = (int)((igrid + nsm - 1) / nsm);
     const size_t slotBytes = sizeof(double) * RING_NF_MAX * ib;
     int depth = (int)((size_t)200 * 1024 / ((size_t)(blocksPerSm < 1 ? 1 : blocksPerSm) * slotBytes)) - 1;
     // the depth is a compile-time constant of the kernel: largest instantiated value that fits
     void (*stepKernel)(Ctx);
-    static const bool stepBulk = []() { const char* e = getenv("MSEETC_STEP_BULK"); return e && atoi(e) != 0; }();
     if (ib == 32) {
         // prefetch depth 16 measured slightly better than 8 (sweep launch 157 -> 153 us: the forward sweep spends ~0.15 us per
-        // interval, so 8 intervals of look-ahead do not cover the DRAM latency under load); MSEETC_STEP_DEPTH=8 selects the old ring
-        static const int stepDepth = []() { const char* e = getenv("MSEETC_STEP_DEPTH"); return e ? atoi(e) : 16; }();
-        if (depth >= 16 && stepDepth >= 16 && !stepBulk) { depth = 16; stepKernel = k_step<32, 16, false>; }
-        else if (depth >= 8) { depth = 8; stepKernel = stepBulk ? k_step<32, 8, true> : k_step<32, 8, false>; }
-        else { depth = 4; stepKernel = k_step<32, 4, false>; }
+        // interval, so 8 intervals of look-ahead do not cover the DRAM latency under load)
+        if (depth >= 16) { depth = 16; stepKernel = k_step<32, 16>; }
+        else if (depth >= 8) { depth = 8; stepKernel = k_step<32, 8>; }
+        else { depth = 4; stepKernel = k_step<32, 4>; }
     } else {
-        if (depth >= 4) { depth = 4; stepKernel = k_step<64, 4, false>; }
-        else if (depth >= 2) { depth = 2; stepKernel = k_step<64, 2, false>; }
-        else { depth = 1; stepKernel = k_step<64, 1, false>; }
+        if (depth >= 4) { depth = 4; stepKernel = k_step<64, 4>; }
+        else if (depth >= 2) { depth = 2; stepKernel = k_step<64, 2>; }
+        else { depth = 1; stepKernel = k_step<64, 1>; }
     }
-    size_t ringBytes = (size_t)(depth + 1) * slotBytes + (size_t)(ib / 32) * 2 * (depth + 1) * sizeof(unsigned long long);
+    size_t ringBytes = (size_t)(depth + 1) * slotBytes;
     // The sweep blocks are spread over the SMs: the request is padded so that no more than blocksPerSm of them fit on one SM
     // (otherwise the block scheduler packs several of these one-warp, latency-bound blocks onto whatever SM has room while a
     // concurrent stream's interval kernels occupy the others, and they slow each other down: 243 -> 196 us per launch and
-    // 129 k -> 137 k solves/s on the bench workload).  MSEETC_STEP_SMEM_KB overrides the padding (0 = none).
-    static const int stepSmemKb = []() { const char* e = getenv("MSEETC_STEP_SMEM_KB"); return e ? atoi(e) : -1; }();
+    // 129 k -> 137 k solves/s on the bench workload).
     {
         const int bps = blocksPerSm < 1 ? 1 : blocksPerSm;
-        const size_t pad = stepSmemKb >= 0 ? (size_t)stepSmemKb * 1024 : (size_t)228 * 1024 / (bps + 1) + 1024;
+        const size_t pad = (size_t)228 * 1024 / (bps + 1) + 1024;
         if (pad > ringBytes && pad <= (size_t)227 * 1024) ringBytes = pad;
     }
     // the attribute belongs to the kernel, not to this call: handles on other host threads launch the same kernel with other
@@ -722,9 +677,9 @@ int mseetc_solve_batch(mseetc_handle h, int32_t n, const double* params, const i
     int tick = 0;
     // ---- starting point: evaluation, convergence test, barrier parameter
     begin(CLS_EVAL);
-    if (intl) launch_variant(c.irk ? VK_EVAL_INTL_IRK : VK_EVAL_INTL, gridIrk, st, c, io);
-    else if (c.irk) launch_variant(dyn ? VK_EVAL_DYN_IRK : VK_EVAL_IRK, gridIrk, st, c, io);
-    else if (dyn) launch_variant(VK_EVAL_DYN, gridEval, st, c, io); else k_cell_eval<<<gridEval, 128, 0, st>>>(c, io);
+    if (intl) launch_variant(c.irk ? VK_EVAL_INTL_IRK : VK_EVAL_INTL, cgrid, st, c, io);
+    else if (c.irk) launch_variant(dyn ? VK_EVAL_DYN_IRK : VK_EVAL_IRK, cgrid, st, c, io);
+    else if (dyn) launch_variant(VK_EVAL_DYN, cgrid, st, c, io); else k_cell_eval<<<cgrid, 128, 0, st>>>(c, io);
     end(CLS_EVAL);
     begin(CLS_KKT); k_inst_kkt<false><<<rgrid * RED_CL, 32 * RED_WB, 0, st>>>(c); end(CLS_KKT);
     // ---- the tick loop: direction (sweeps, interval-parallel rest, step-size limits), then the evaluation at the trial point with
@@ -733,27 +688,25 @@ int mseetc_solve_batch(mseetc_handle h, int32_t n, const double* params, const i
     // body; the last kernel of the body sets the condition from the completion counter, so the host neither launches the ticks nor
     // polls.  Large batches keep the host loop below: it already runs two ticks ahead of the device, and next to the concurrent
     // minimum-time presolve (a second while-graph on a high-priority stream) the device loop measured slower (30.2 against 23.8 ms
-    // per 4096-instance sweep).  MSEETC_GRAPH=1 / 0 forces the device / host loop; per-kernel profiling needs the host loop.
-    static const bool compactOn = []() { const char* e = getenv("MSEETC_COMPACT"); return !e || atoi(e) != 0; }();
+    // per 4096-instance sweep).  Per-kernel profiling needs the host loop.
     h->last_compactions = 0;
-    static const int graphEnv = []() { const char* e = getenv("MSEETC_GRAPH"); return e ? atoi(e) : -1; }();
-    const bool useGraph = !h->profiling && (graphEnv == 1 || (graphEnv != 0 && g.S <= 256 && !tmin));
+    const bool useGraph = !h->profiling && g.S <= 256 && !tmin;
     auto tick_kernels = [&](cudaStream_t s0, int* mirror, bool prof) {
         if (prof) begin(CLS_STEP);
         if (pitKernel) pitKernel<<<(unsigned)(g.S / pitSL), pitThreads, pitBytes, s0>>>(c, c.done + 48);
         else stepKernel<<<igrid, ib, ringBytes, s0>>>(c);
         if (prof) end(CLS_STEP);
         if (prof) begin(CLS_CSTEP);
-        if (intl) launch_variant(VK_STEP_INTL, pgrid(2), s0, c, io);
-        else if (dyn) launch_variant(VK_STEP_DYN, gridStep, s0, c, io); else k_cell_step<<<gridStep, 128, 0, s0>>>(c, io);
+        if (intl) launch_variant(VK_STEP_INTL, cgrid, s0, c, io);
+        else if (dyn) launch_variant(VK_STEP_DYN, cgrid, s0, c, io); else k_cell_step<<<cgrid, 128, 0, s0>>>(c, io);
         if (prof) end(CLS_CSTEP);
         if (prof) begin(CLS_ALPHA);
         k_inst_alpha<<<rgrid * RED_CL, 32 * RED_WB, 0, s0>>>(c, mirror);
         if (prof) end(CLS_ALPHA);
         if (prof) begin(CLS_TRIAL);
-        if (intl) launch_variant(c.irk ? VK_TRIAL_INTL_IRK : VK_TRIAL_INTL, gridIrk, s0, c, io);
-        else if (c.irk) launch_variant(dyn ? VK_TRIAL_DYN_IRK : VK_TRIAL_IRK, gridIrk, s0, c, io);
-        else if (dyn) launch_variant(VK_TRIAL_DYN, gridTrial, s0, c, io); else k_cell_trial_eval<<<gridTrial, 128, 0, s0>>>(c, io);
+        if (intl) launch_variant(c.irk ? VK_TRIAL_INTL_IRK : VK_TRIAL_INTL, cgrid, s0, c, io);
+        else if (c.irk) launch_variant(dyn ? VK_TRIAL_DYN_IRK : VK_TRIAL_IRK, cgrid, s0, c, io);
+        else if (dyn) launch_variant(VK_TRIAL_DYN, cgrid, s0, c, io); else k_cell_trial_eval<<<cgrid, 128, 0, s0>>>(c, io);
         if (prof) end(CLS_TRIAL);
         if (prof) begin(CLS_DECIDE);
         k_inst_kkt<true><<<rgrid * RED_CL, 32 * RED_WB, 0, s0>>>(c);
@@ -818,7 +771,7 @@ int mseetc_solve_batch(mseetc_handle h, int32_t n, const double* params, const i
                 if (doneLag >= n) break;
                 // compaction (compact.cuh): every fourth tick once instances have finished; the plan kernel decides on the device
                 // whether the running instances are scattered enough to be worth moving, the other kernels return at once if not
-                if (compactOn && h->compaction && !intl && g.S >= 256 && doneLag > 0 && tick % 4 == 0) {
+                if (h->compaction &&!intl && g.S >= 256 && doneLag > 0 && tick % 4 == 0) {
                     const int activeUb = n - doneLag;
                     k_compact_plan<<<1, 1024, 0, st>>>(c);
                     k_compact_extract<<<cgrid, 128, 0, st>>>(c, io);

@@ -76,14 +76,13 @@ MS_HD bool chunk_element_t(const Ctx& c, int s, int kLo, int kHi, double mu, dou
     E.Phi[0] = E.Phi[4] = E.Phi[8] = 1.0;
     for (int i = 0; i < 3; ++i) E.phi[i] = 0.0;
     for (int i = 0; i < 6; ++i) E.W[i] = 0.0;
-    bool ok = true;
     if (kHi > kLo) {
         fetch.start(c, s, kHi - 1, kLo, -1);
         for (int k = kHi - 1; k >= kLo; --k) {
             double v[BwdFields::NF], vs[6], K[3][3], kf[3], cb[4];
             fetch.get(c, k, s, v);
             if (REG) load_scol(c, k, s, vs);
-            if (!stage_riccati_sparse(v, REG ? vs : nullptr, mu, delta, pn, P, p, K, kf, cb)) { ok = false; if (!Fetch::COLLECTIVE) return false; }
+            if (!stage_riccati_sparse(v, REG ? vs : nullptr, mu, delta, pn, P, p, K, kf, cb)) return false;
             const double tb = v[QP_TAU_B], tF = v[QP_TAU_F], pb = v[QP_PHI_B], pF = v[QP_PHI_F];
             // Gramian: W += Y Rt^{-1} Y',  Y = Phi_{e<-k+1} B,  B = [(tF, pF, 1)  pn (tF, pF, 0)]
             double yF[3], yQ[3], xF[3], xQ[3];
@@ -109,7 +108,7 @@ MS_HD bool chunk_element_t(const Ctx& c, int s, int kLo, int kHi, double mu, dou
     }
     full_to_sym(P, E.P);
     for (int i = 0; i < 3; ++i) E.p[i] = p[i];
-    return ok;
+    return true;
 }
 template <class Fetch>
 MS_HD bool chunk_element(const Ctx& c, int s, int kLo, int kHi, double mu, double delta, Fetch& fetch, const double* refP, const double* refp,

@@ -27,24 +27,18 @@ namespace mseetc {
 // of k+1 follows at a compile-time stride, so the address arithmetic of a sweep is one pointer bump per interval.
 enum { REC_STRIDE = WS_FIELDS * 32 };
 struct BwdFields {   // condensed stage Hessian (9), linearised coupling rows (6), condensed gradient parts (4 + 4)
-    enum { NF = QP_SWEEP_N, NRANGE = 1 };
+    enum { NF = QP_SWEEP_N };
     static MS_HD constexpr int off(int f) { return (WS_QP + f) * 32; }
-    // contiguous field ranges of a (tile, k) record, for bulk copies: first field, number of fields
-    static MS_HD constexpr int range_first(int) { return WS_QP; }
-    static MS_HD constexpr int range_count(int) { return QP_SWEEP_N; }
 };
 struct FwdFields {   // feedback rows of Fel, Fpb (6 + 2) | linearised coupling rows (6)
-    enum { NF = 14, NRANGE = 2 };
+    enum { NF = 14 };
     static MS_HD constexpr int off(int f) { return f < 8 ? (WS_RIC + RIC_K + f) * 32 : (WS_QP + QP_TAU_B + (f - 8)) * 32; }
-    static MS_HD constexpr int range_first(int r) { return r == 0 ? WS_RIC + RIC_K : WS_QP + QP_TAU_B; }
-    static MS_HD constexpr int range_count(int r) { return r == 0 ? 8 : 6; }
 };
 enum { RING_NF_MAX = QP_SWEEP_N };
 
 // direct loads (host emulation, and the device when no ring is configured)
 template <class FL>
 struct DirectFetch {
-    enum { COLLECTIVE = 0 };
     MS_HD void start(const Ctx&, int, int, int, int) {}
     MS_HD void get(const Ctx& c, int k, int s, double* v) {
         const double* rec = &c.W(0, k, s);
@@ -61,7 +55,6 @@ struct DirectFetch {
 // registers), so that a shallow ring sees L2 latency instead of DRAM latency
 template <class FL, int BS, int DEPTH, int PF = 0>
 struct RingFetch {
-    enum { COLLECTIVE = 0 };
     double* sm;          // this thread's column of slot 0
     const double* next;  // record of the next interval to request
     int left;            // intervals not yet requested
@@ -99,92 +92,6 @@ struct RingFetch {
         const double* src = sm + head * (FL::NF * BS);
 #pragma unroll
         for (int f = 0; f < FL::NF; ++f) v[f] = src[f * BS];
-        head = (head == DEPTH) ? 0 : head + 1;
-        issue();
-    }
-};
-
-// Bulk-copy ring (TMA unit, cp.async.bulk + mbarrier): when all running instances of a warp's tile have the same interval
-// count they walk the intervals together, and the stage data of the whole tile -- contiguous in the tiled layout -- is
-// fetched by ONE bulk copy per field range issued by one lane, completion signalled on a shared-memory mbarrier.
-// DEPTH + 1 slots; a slot is refilled one iteration after the warp has copied it to registers (__syncwarp in between).
-namespace bulk {
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_init_fence() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void copy_g2s(void* dst, const void* src, unsigned bytes, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-    unsigned done;
-    do {
-        asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-                     : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    } while (!done);
-}
-}  // namespace bulk
-
-template <class FL, int DEPTH>
-struct BulkRing {
-    enum { COLLECTIVE = 1 };    // all running lanes of the warp must consume every requested interval
-    double* sm;                 // ring of this warp: slot stride FL::NF * 32 doubles, field-major, lane-minor
-    unsigned long long* bar;    // DEPTH + 1 mbarriers of this warp and this field list
-    const double* next;         // (tile, k) record of the next interval to request
-    long step;
-    int left, head, tail, lane;
-    unsigned phase, mask;
-    bool leader;
-    __device__ void setup(double* ringBase, unsigned long long* bars, unsigned activeMask, int laneId) {
-        sm = ringBase; bar = bars; mask = activeMask; lane = laneId; phase = 0u;
-        leader = (laneId == __ffs((int)activeMask) - 1);
-        if (leader) {
-            for (int i = 0; i <= DEPTH; ++i) bulk::mbar_init(bar + i, 1);
-            bulk::mbar_init_fence();
-        }
-        __syncwarp(mask);
-    }
-    __device__ void issue() {
-        if (left > 0) {
-            if (leader) {
-                bulk::mbar_expect_tx(bar + tail, (unsigned)(FL::NF * 32 * sizeof(double)));
-                double* dst = sm + tail * (FL::NF * 32);
-#pragma unroll
-                for (int r = 0; r < FL::NRANGE; ++r) {
-                    bulk::copy_g2s(dst, next + FL::range_first(r) * 32, (unsigned)(FL::range_count(r) * 32 * sizeof(double)), bar + tail);
-                    dst += FL::range_count(r) * 32;
-                }
-            }
-            next += step;
-            --left;
-        }
-        tail = (tail == DEPTH) ? 0 : tail + 1;
-    }
-    __device__ void start(const Ctx& c, int s, int kFirst, int kLast, int direction) {
-        // the forward sweep fetches what the lanes of this warp stored in the backward sweep: order those generic-proxy
-        // stores before the async-proxy reads of the copy unit, then meet the issuing lane
-        __threadfence();
-        asm volatile("fence.proxy.async;" ::: "memory");
-        __syncwarp(mask);
-        next = &c.W(0, kFirst, s & ~31);
-        step = (long)direction * REC_STRIDE;
-        left = (direction < 0 ? kFirst - kLast : kLast - kFirst) + 1;
-        head = tail = 0;
-#pragma unroll
-        for (int d = 0; d < DEPTH; ++d) issue();
-    }
-    __device__ void get(const Ctx&, int, int, double* v) {
-        bulk::mbar_wait(bar + head, (phase >> head) & 1u);
-        phase ^= 1u << head;
-        const double* src = sm + head * (FL::NF * 32) + lane;
-#pragma unroll
-        for (int f = 0; f < FL::NF; ++f) v[f] = src[f * 32];
-        __syncwarp(mask);          // every lane has its copy: the slot consumed one iteration ago may be refilled
         head = (head == DEPTH) ? 0 : head + 1;
         issue();
     }
@@ -435,11 +342,8 @@ MS_HD bool riccati_backward_range_t(const Ctx& c, int s, int N, int kLo, int kHi
     if (kHi <= kLo) return true;
     fetch.start(c, s, kHi - 1, kLo, -1);
     int k = kHi - 1;
-    // with a ring that is collective over the warp a failed inertia test does not leave the loop (every requested interval has
-    // to be consumed; the remaining, discarded stages cost one sweep in the rare regularisation case); otherwise it returns at once
-    bool ok = true;
+    // a failed inertia test leaves the sweep at once (copies still in flight are drained by the next fetch.start)
     double v[BwdFields::NF], K[3][3], kf[3];
-    if (Fetch::COLLECTIVE) for (int i = 0; i < 3; ++i) { kf[i] = 0.0; for (int j = 0; j < 3; ++j) K[i][j] = 0.0; }
     if (k == N - 1) {
         // last interval: terminal speed fixed, Fel eliminated (dense algebra, once per sweep)
         fetch.get(c, k, s, v);
@@ -447,7 +351,7 @@ MS_HD bool riccati_backward_range_t(const Ctx& c, int s, int N, int kLo, int kHi
         load_scol(c, k, s, vs);
         StageQP q;
         stage_build(v, vs, mu, delta, pn, true, q);
-        if (!stage_riccati(q, true, pn, P, p, K, kf)) { if (!Fetch::COLLECTIVE) return false; ok = false; }
+        if (!stage_riccati(q, true, pn, P, p, K, kf)) return false;
         if (storeAll || k == kLo) stage_store(c, k, s, K, kf, P, p);
         if (Mc) {
             double Mk[9], mk[3];
@@ -463,7 +367,7 @@ MS_HD bool riccati_backward_range_t(const Ctx& c, int s, int N, int kLo, int kHi
         fetch.get(c, k, s, v);
         double vs[6];
         if (REG) load_scol(c, k, s, vs);
-        if (!stage_riccati_sparse(v, REG ? vs : nullptr, mu, delta, pn, P, p, K, kf)) { if (!Fetch::COLLECTIVE) return false; ok = false; }
+        if (!stage_riccati_sparse(v, REG ? vs : nullptr, mu, delta, pn, P, p, K, kf)) return false;
         if (storeAll || k == kLo) stage_store(c, k, s, K, kf, P, p);
         if (Mc) {
             const double tb = v[QP_TAU_B], tF = v[QP_TAU_F], pb = v[QP_PHI_B], pF = v[QP_PHI_F];
@@ -479,14 +383,13 @@ MS_HD bool riccati_backward_range_t(const Ctx& c, int s, int N, int kLo, int kHi
             closed_loop_compose(Mc, mc, Mk, mk);
         }
     }
-    return ok;
+    return true;
 }
 
 template <class Fetch>
 MS_HD bool riccati_backward_range(const Ctx& c, int s, int N, int kLo, int kHi, double mu, double delta, Fetch& fetch,
                                   double P[3][3], double p[3], double* Mc, double* mc, bool storeAll = true) {
-    // a collective ring keeps all lanes of the warp in one variant (the correction terms vanish for delta = 0)
-    if (Fetch::COLLECTIVE || delta > 0.0) return riccati_backward_range_t<true>(c, s, N, kLo, kHi, mu, delta, fetch, P, p, Mc, mc, storeAll);
+    if (delta > 0.0) return riccati_backward_range_t<true>(c, s, N, kLo, kHi, mu, delta, fetch, P, p, Mc, mc, storeAll);
     return riccati_backward_range_t<false>(c, s, N, kLo, kHi, mu, delta, fetch, P, p, Mc, mc, storeAll);
 }
 
@@ -668,42 +571,6 @@ MS_HD void inst_step(const Ctx& c, int s, FetchB& fb, FetchF& ff) {
     c.I(SI_FACT, s) = 1;
     c.I(SI_PHASE, s) = PH_STEPPED;
 }
-
-#if defined(__CUDACC__)
-// The same for a warp whose running lanes walk the intervals together (collective prefetch ring): lanes whose factorisation
-// already succeeded repeat the backward sweep with their own (unchanged) delta -- same result -- while others regularise.
-template <class FetchB, class FetchF>
-__device__ void inst_step_warp(const Ctx& c, int s, unsigned mask, FetchB& fb, FetchF& ff) {
-    const int N = c.I(SI_N_INT, s);
-    const double mu = c.D(SD_MU, s);
-    double delta = 0.0;
-    const double dlast = c.D(SD_DELTA_LAST, s);
-    bool ok = false, dead = false;
-    for (int tries = 0; tries < 40; ++tries) {
-        const bool run = !ok && !dead;
-        if (run) count_cells(c, 2, N);
-        const bool r = riccati_backward(c, s, N, mu, delta, fb);
-        if (run) {
-            if (r) ok = true;
-            else {
-                c.I(SI_NREG, s) += 1;
-                if (delta == 0.0) delta = (dlast == 0.0) ? 1e-4 : fmax(1e-20, dlast / 3.0);
-                else delta *= (dlast == 0.0) ? 100.0 : 8.0;
-                if (delta > 1e40) dead = true;
-            }
-        }
-        if (!__any_sync(mask, !ok && !dead)) break;
-    }
-    if (ok) {
-        if (delta > 0.0) c.D(SD_DELTA_LAST, s) = delta;
-        c.D(SD_DELTA, s) = delta;
-        count_cells(c, 3, N);
-    }
-    riccati_forward(c, s, N, mu, delta, ff);
-    if (ok) c.I(SI_PHASE, s) = PH_STEPPED;
-    else finish(c, s, ST_STEP_FAILED);
-}
-#endif
 
 // ---- interval-parallel part of the step --------------------------------------------------------------------
 // fraction-to-boundary limits of one cell, kept as fractions: the smallest ratio slack / (-d slack) (and z / (-d z)) of the bounds

@@ -27,6 +27,9 @@ inline void launch_variant(int which, unsigned grid, cudaStream_t st, const Ctx&
 // mseetc_eval_interval with collocation steps (`irk`: device pointer)
 void launch_eval_interval_irk(int n, int numSteps, int numApprox, const double* in, double* out, const IrkTab* irk, cudaStream_t st);
 
+// minimum resident blocks per SM of k_cell_step and k_cell_step_dyn (3 measured faster than 2 or 4)
+enum { CELL_STEP_MINB = 3 };
+
 #define MS_CELL_KERNEL(NAME, MINB, CALL)                                        \
     __global__ void __launch_bounds__(128, MINB) NAME(Ctx c, BatchIO io) {      \
         const size_t total = (size_t)c.cfg.NK * c.cfg.S;                        \

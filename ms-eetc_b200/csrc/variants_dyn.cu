@@ -3,14 +3,11 @@
 
 namespace mseetc {
 namespace {
-#ifndef MS_MINB_STEP
-#define MS_MINB_STEP 3
-#endif
 // the row gradients of the loss rows come from the stage-QP record (see cell_step)
 MS_CELL_KERNEL(k_cell_init_dyn, 2, cell_init<true>(c, k, s))
 MS_CELL_KERNEL(k_cell_trial_eval_dyn, 2, (cell_eval<true, true>(c, k, s)))
 MS_CELL_KERNEL(k_cell_eval_dyn, 2, (cell_eval<true, false>(c, k, s)))
-MS_CELL_KERNEL(k_cell_step_dyn, MS_MINB_STEP, cell_step<true>(c, k, s))
+MS_CELL_KERNEL(k_cell_step_dyn, CELL_STEP_MINB, cell_step<true>(c, k, s))
 }  // namespace
 
 void launch_variant_dyn(int which, unsigned grid, cudaStream_t st, const Ctx& c, const BatchIO& io) {

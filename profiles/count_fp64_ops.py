@@ -32,7 +32,7 @@ for cls, sub in (('cell_trial', 'k_cell_trial_evalE'), ('cell_eval', 'k_cell_eva
                  ('cell_trial_dyn', 'k_cell_trial_eval_dynE'), ('cell_eval_dyn', 'k_cell_eval_dynE')):
     f, n = flops(funcs[find(sub)[0]])
     out[cls] = {'flop_per_cell': f, 'instructions': n}
-ks = funcs[[k for k in find('k_stepILi32ELi8ELb0E')][0]]
+ks = funcs[[k for k in find('k_stepILi32ELi8EE')][0]]
 loops = []
 for a, t in ks:
     m = re.search(r'BRA\s+(?:U?P\d,\s*)?(0x[0-9a-f]+)', t)
